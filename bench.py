@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the UNMODIFIED reference command line on the host cores
+    python bench.py ... --dump-outputs DIR                   # + the rows of the last timed step, to compare two builds
 
 Workload (BASELINE.json configs[1], "C2"): 4 populations x 50 diploid samples (H = 400 haplotypes), 10 M synthetic sites per
 GPU, -w 50000 coordinate windows (~5000 sites each), -m 100, minData 0.01.  A "step" is one pass of the hot path (site pass ->
@@ -297,6 +298,28 @@ def rows_equal(a: dict, b: dict, keys, rtol=0.0):
     return True
 
 
+DUMP_KEYS = ("sites", "pos_sum", "path", "pi", "dxy", "fst")
+DUMP_LIMIT = 60_000_000          # bytes of array data: the files stay below 64 MB, .npy headers included
+
+
+def dump_outputs(directory, legs, limit=DUMP_LIMIT):
+    """Window rows of the last timed step of each leg as <directory>/<leg>_<key>.npy (float64; the integer columns are
+    below 2**53).  Past `limit` bytes in all, every leg keeps a seeded sample of its windows, listed in <leg>_window.npy."""
+    os.makedirs(directory, exist_ok=True)
+    total = sum(np.asarray(rows[k]).size * 8 for rows in legs.values() for k in DUMP_KEYS)
+    scale = limit / (total + 8 * sum(len(rows["sites"]) for rows in legs.values()))     # + the window index
+    for leg, rows in legs.items():
+        W = len(rows["sites"])
+        keep = None
+        if total > limit:
+            n = max(1, int(W * scale))
+            keep = np.sort(np.random.default_rng(SEED).choice(W, size=n, replace=False))
+            np.save(os.path.join(directory, "%s_window.npy" % leg), keep.astype(np.float64))
+        for k in DUMP_KEYS:
+            a = np.asarray(rows[k], dtype=np.float64)
+            np.save(os.path.join(directory, "%s_%s.npy" % (leg, k)), a if keep is None else a[keep])
+
+
 def main():
     quiet_stdout()
     ap = argparse.ArgumentParser()
@@ -308,6 +331,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-legs", action="store_true", help="skip the C3 / C4 / C5 / text legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the window rows of the last timed step of the two C2 legs as DIR/<name>.npy (float64)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -443,12 +468,14 @@ def main():
         intervals.append((t0, t0 + dtp_local))
         dt_pipe = max_over_ranks(dtp_local)
         launches_pipe = eng.launch_count() - l0
+        last = np.array(last)                        # the slot is pinned memory that later batches overwrite
         ref_tab = step()
         if dist is not None:
-            pipe_equal = bool(np.array_equal(np.asarray(last).view(np.uint64), np.asarray(ref_tab).view(np.uint64)))
+            pipe_equal = bool(np.array_equal(last.view(np.uint64), np.asarray(ref_tab).view(np.uint64)))
+            out_rows = multigpu.unpack_device_records(multigpu.gathered_rows(last, counts, w_max), P)
         else:
-            mine = multigpu.unpack_device_records(np.asarray(last)[:len(lo)], P)
-            pipe_equal = rows_equal(ref_tab, mine, ("sites", "pos_sum", "path", "pi", "dxy", "fst"))
+            out_rows = multigpu.unpack_device_records(last[:len(lo)], P)
+            pipe_equal = rows_equal(ref_tab, out_rows, ("sites", "pos_sum", "path", "pi", "dxy", "fst"))
         # correctness of the gathered rows: rank 0 recomputes every rank's shard alone
         equal = None
         if dist is not None:
@@ -471,7 +498,8 @@ def main():
             barrier()
         paths = np.bincount(eng.popgen(MIN_SITES, MIN_DATA)["path"], minlength=3).tolist()
         return dict(dt=dt, tms=tms, launches=launches, steps=steps, W=len(lo), lo=lo, hi=hi, step=step, equal=equal,
-                    paths=paths, table=table, dt_pipe=dt_pipe, launches_pipe=launches_pipe, pipe_equal=pipe_equal)
+                    paths=paths, table=table, dt_pipe=dt_pipe, launches_pipe=launches_pipe, pipe_equal=pipe_equal,
+                    out_rows=out_rows)
 
     A = c2_leg(0.0, args.steps, args.warmup)
     value_sync = world * S * args.steps / A["dt"]
@@ -834,6 +862,8 @@ def main():
             "paths_missing": {"failed": B["paths"][0], "closed_form_K1": B["paths"][1], "pairwise_K2": B["paths"][2]},
             "c3": legs.get("c3"), "c4": legs.get("c4"), "c5": legs.get("c5"), "from_text": legs.get("from_text"),
             "variants": variants}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"c2": A["out_rows"], "c2_missing": B["out_rows"]})
     emit(line)
     eng.close()
     if dist is not None:
